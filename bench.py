@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — CPR head img/s @1333x800 (BASELINE.json metric) on N B200s + HBM roofline of the neighbor gather.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Step = one pass of the CPR head over one batch of synthetic FPN tensors: CPRHead.simple_test == forward (4x conv3x3+GN+
@@ -349,7 +349,11 @@ def main():
     ap.add_argument('--p2p-train', action='store_true', help='also time a P2PHead training step (its two narrow output convs run on cuDNN under '
                     'autograd: the first cuDNN use pages the library in, minutes on a cold box)')
     ap.add_argument('--profile', action='store_true', help='for runs under ncu: no load-holding steps, no e2e, no extras')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the detections of the last timed step (rank 0) to DIR/*.npy, so that two '
+                    'builds can be compared output for output on the same seeded inputs')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -451,7 +455,7 @@ def main():
         l0 = ops.launch_count()
         e0.record()
         for i in range(steps):
-            fn(i)
+            out = fn(i)
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
@@ -460,7 +464,7 @@ def main():
         t = torch.tensor([ms], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t[0]), launches
+        return float(t[0]), launches, out
 
     sampler = ClockSampler(local)
     if rank == 0:
@@ -471,11 +475,17 @@ def main():
         step_resident(i)
     wall = {'setup': time.perf_counter() - T_MAIN}
     t_begin = time.perf_counter()
-    ms, launches = timed(step_resident, args.steps)
+    ms, launches, last_out = timed(step_resident, args.steps)
     wall['timed_steps'] = time.perf_counter() - T_MAIN
     t_end = time.perf_counter()
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
     value = world * B * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        # what CPRHead.simple_test hands its caller, per image: dets (n, 6) = [x1, y1, x2, y2, score, ann_id] and labels (n,);
+        # every image has CFG['n'] points, so the images stack.  96 KB in all at the default workload.
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, 'dets.npy'), torch.stack([d for d, _ in last_out]).cpu().numpy().astype(np.float32))
+        np.save(os.path.join(args.dump_outputs, 'labels.npy'), torch.stack([l for _, l in last_out]).cpu().numpy().astype(np.float64))
 
     if args.profile:
         if rank == 0:
