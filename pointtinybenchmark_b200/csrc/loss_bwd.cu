@@ -11,8 +11,9 @@
 //   A  the bags of the image whose sample window reaches the tile, in GT order (ordered ballot compaction);
 //   B  bag by bag, warp w evaluates samples 32w .. 32w+31 (lane = sample: tap geometry, which taps land in the tile) and the samples
 //      with a tap in the tile are appended to a record buffer in (bag, k) order;
-//   C  rounds of 64 records: (1) one warp per record, lanes = classes: two coalesced loads of the sampled logits, the per-sample gradient
-//      row staged in shared memory; (2) the <= 256 (record, tap) hits of the round are counting-sorted by cell (stable); (3) every
+//   C  rounds of min(64, blockDim.x / 4) records: (1) one warp per record, lanes = classes: two coalesced loads of the sampled logits,
+//      the per-sample gradient row staged in shared memory; (2) the <= blockDim.x (record, tap) hits of the round are counting-sorted by
+//      cell (stable), one thread per hit; (3) every
 //      (cell, channel group) thread walks its cell's hits in order: acc += w * staged row.
 // No atomics anywhere and every sum is evaluated by ONE thread in a FIXED order: bit-identical run to run, no zero-initialised gradient
 // map, no materialised (G,K,2N) gradient tensor (740 MB written and re-read in round 1).  ncu history: a first version (one warp per
@@ -93,11 +94,13 @@ cpr_loss_bwd_tile_kernel(const LossBwdArgs a) {
   for (int i = tid; i < LB_ROUND * LDS; i += blockDim.x) st[i] = 0.f;      // pad columns [N, NP) stay zero for the whole kernel
   if (tid == 0) s_nrec = 0;
 
-  // ---- C: consume the record buffer in rounds of LB_ROUND
+  // ---- C: consume the record buffer in rounds of up to LB_ROUND records.  Step (2) ranks each (record, tap) hit on the thread of the
+  // same index, so a round holds at most blockDim.x / 4 records: 64 at LD >= 128, 16 / 32 / 48 at LD 32 / 64 / 96
+  const int per_round = min(LB_ROUND, (int)blockDim.x / 4);
   auto process = [&]() {
     const int nrec = s_nrec;                                               // (caller has synchronised)
-    for (int r0 = 0; r0 < nrec; r0 += LB_ROUND) {
-      const int nr = min(LB_ROUND, nrec - r0);
+    for (int r0 = 0; r0 < nrec; r0 += per_round) {
+      const int nr = min(per_round, nrec - r0);
       // (1) gradient rows: one warp per record, lanes = classes
       for (int r = warp; r < nr; r += nwarps) {
         const LbRec rec = s_rec[r0 + r];
@@ -386,7 +389,14 @@ extern "C" int ptb_cpr_loss_bwd_map(const float* bag_logits, const float* weight
   const int threads = LB_CELLS * (ld / 32);
   PTB_REQUIRE(threads <= 320 || ld <= 512, "ld");
   if (threads > 320) return fail("%s", "ptb_cpr_loss_bwd_map: ld > 160 needs more than 320 threads per tile (not built)");
-  if (smem > 40 * 1024 &&
+  // the kernel's static shared memory (record buffer, candidates, hit list: ~21 KB) counts against the 48 KB that need no opt-in
+  static int static_smem = -1;
+  if (static_smem < 0) {
+    cudaFuncAttributes fa;
+    if (cudaFuncGetAttributes(&fa, cpr_loss_bwd_tile_kernel) != cudaSuccess) return fail("%s", "ptb_cpr_loss_bwd_map: cudaFuncGetAttributes failed");
+    static_smem = (int)fa.sharedSizeBytes;
+  }
+  if (static_smem + smem > 48 * 1024 &&
       cudaFuncSetAttribute(cpr_loss_bwd_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return fail("%s", "ptb_cpr_loss_bwd_map: shared memory opt-in failed");
   dim3 grid((W + LB_T - 1) / LB_T, (H + LB_T - 1) / LB_T, B);

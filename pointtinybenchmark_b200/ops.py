@@ -341,13 +341,17 @@ def mil_loss_bwd(logits, num_classes, ins_off, weight, labels, eps, bag_prob, sc
 
 
 def cpr_loss_bwd_map(bag_logits, weight, mil_mt, bag_prob, label_weight, labels, centers, img_ptr, offsets, map_shape, num_classes, ins_off,
-                     stride, reach_px, eps, scale_mil=None, scale_gt=None, valid_center=None, logit_map=None, neg_mask=None, scale_neg=None):
-    """ptb_cpr_loss_bwd_map: d loss / d logit map (B,H,W,ld), deterministic, every element written."""
+                     stride, reach_px, eps, scale_mil=None, scale_gt=None, valid_center=None, logit_map=None, neg_mask=None, scale_neg=None,
+                     out=None):
+    """ptb_cpr_loss_bwd_map: d loss / d logit map (B,H,W,ld), deterministic, every element written (into `out` when given)."""
     lib = _lib.load()
     _chk(bag_logits, torch.float32, 'bag_logits'); _chk(weight, torch.float32, 'weight'); _chk(centers, torch.float32, 'centers')
     B, H, W, ld = map_shape
     G, K, _ = bag_logits.shape
-    out = torch.empty((B, H, W, ld), dtype=torch.float32, device=bag_logits.device)
+    if out is None:
+        out = torch.empty((B, H, W, ld), dtype=torch.float32, device=bag_logits.device)
+    elif tuple(_chk(out, torch.float32, 'out').shape) != (B, H, W, ld):
+        raise ValueError(f'out: expected shape {(B, H, W, ld)}, got {tuple(out.shape)}')
     ws = torch.empty(int(lib.ptb_cpr_loss_bwd_map_workspace(G, num_classes)) // 4, dtype=torch.float32, device=bag_logits.device)
     check(lib.ptb_cpr_loss_bwd_map(_ptr(bag_logits), _ptr(weight), _ptr(mil_mt), _ptr(bag_prob), _ptr(label_weight), _ptr(labels),
                                    _ptr(centers), _ptr(img_ptr), _ptr(offsets), B, H, W, G, K, num_classes, ins_off, ld, float(stride),
