@@ -448,6 +448,36 @@ int ptb_conv_tc_wgrad_f16x2(const void* dy_h, const void* dy_l /*[B][H][W][Cout]
 uint64_t ptb_col_sum_workspace(int64_t M, int N);
 int ptb_col_sum(const float* y /*[M][ld]*/, int64_t M, int N, int ld, float* workspace, float* out /*[N]*/, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * R-CNN box stage (StandardRoIHead.simple_test_bboxes with SingleRoIExtractor + Shared2FCBBoxHead; roi_heads/test_mixins.py:50-130,
+ * single_level_roi_extractor.py:34-100, bbox_head.py:310-435).
+ *   ptb_amax_abs          max|x| of an fp32 tensor as float bits into *dev_amax_bits (atomicMax over non-negative floats); accumulate = 0
+ *                         zeroes it first, 1 keeps the running max (several levels into one bound).
+ *   ptb_roi_align         rois (M, 5) [batch_idx, x1, y1, x2, y2]; L <= 5 channels-last fp32 level maps (B, H_l, W_l, C), C % 32 == 0,
+ *                         given as host arrays feats[L], hw[2L] (H, W), spatial_scales[L].  Level per RoI = map_roi_levels (finest_scale;
+ *                         L == 1: level 0), mmcv RoIAlign avg pooling (aligned: offset 0.5, else roi size >= 1; sampling_ratio 0 = adaptive).
+ *                         Exactly one output mode: out (M, out_h, out_w, C) fp32, or out_h16 / out_l16 (M_pad, out_h*out_w*C) fp16 pair of
+ *                         x * s with s the power-of-two scale of ptb_split_f16_amax taken from *dev_amax_bits (1/s -> *dev_inv_scale;
+ *                         rows M .. M_pad-1 are zero).  out_level (M,) int8 optional (-1: NaN scale, features zero).
+ *   ptb_relu_split_f16    y (rows, ld) fp32 -> fp16 pair of relu(y[:, :n]) at unit scale; values above 60000 are clamped and raise
+ *                         *overflow_flag (optional).
+ *   ptb_rcnn_bbox_decode  rois (B * n_per_img, 5), logits cls (rows, ldc) with N + 1 columns, deltas reg (rows, ldr) with 4N columns:
+ *                         mask_padding zeroes logits and deltas of all-zero RoIs (the batch padding of simple_test_bboxes); softmax;
+ *                         class-specific delta2bbox (means, stds, wh_ratio_clip) clipped to img_hw (B, 2) int32 (h, w); rescale by
+ *                         scale_factor (B, 4) when given.  out_boxes (rows, 4N); out_scores (rows, N + 1) and out_cand_scores
+ *                         (rows * N, N): the candidate (RoI i, class k) has its score in column k and -inf elsewhere, the input of
+ *                         ptb_multiclass_nms_boxes with P = n_per_img * N.  Both optional.
+ */
+int ptb_amax_abs(const float* x, int64_t n, unsigned int* dev_amax_bits, int accumulate, void* stream);
+int ptb_roi_align(const float* rois, int M, int M_pad, const void* const* feats, const int32_t* hw, const float* spatial_scales, int L, int B,
+                  int C, int out_h, int out_w, int sampling_ratio, int aligned, float finest_scale, const unsigned int* dev_amax_bits,
+                  float* out, void* out_h16, void* out_l16, float* dev_inv_scale, int8_t* out_level, void* stream);
+int ptb_relu_split_f16(const float* y, int rows, int n, int ld, void* out_h, void* out_l, int* overflow_flag, void* stream);
+int ptb_rcnn_bbox_decode(const float* rois, int B, int n_per_img, const float* cls, int ldc, const float* reg, int ldr, int num_classes,
+                         int mask_padding, const float* means /*host [4]*/, const float* stds /*host [4]*/, float wh_ratio_clip,
+                         const int32_t* img_hw, const float* scale_factor /*or NULL*/, float* out_boxes, float* out_scores /*or NULL*/,
+                         float* out_cand_scores /*or NULL*/, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -91,6 +91,10 @@ SIGNATURES = {
     'ptb_conv_tc_wgrad_f16x2': (c_int, [P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_float, P, P, P, P, c_int, P]),
     'ptb_col_sum_workspace': (c_u64, [c_i64, c_int]),
     'ptb_col_sum': (c_int, [P, c_i64, c_int, c_int, P, P, P]),
+    'ptb_amax_abs': (c_int, [P, c_i64, P, c_int, P]),
+    'ptb_roi_align': (c_int, [P, c_int, c_int, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, P, P, P, P, P, P, P]),
+    'ptb_relu_split_f16': (c_int, [P, c_int, c_int, c_int, P, P, P, P]),
+    'ptb_rcnn_bbox_decode': (c_int, [P, c_int, c_int, P, c_int, P, c_int, c_int, c_int, P, P, c_float, P, P, P, P, P, P]),
 }
 
 

@@ -8,7 +8,7 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(os.path.dirname(HERE), 'libptb_b200.so')
-SOURCES = ['capi.cu', 'gather.cu', 'linear.cu', 'negmask.cu', 'refine.cu', 'gridbag.cu', 'mil.cu', 'p2p.cu', 'nms.cu', 'conv_tc.cu', 'tower_bwd.cu', 'wgrad_tc.cu', 'assign.cu', 'lsap.cu', 'rpn.cu', 'loss_bwd.cu']
+SOURCES = ['capi.cu', 'gather.cu', 'linear.cu', 'negmask.cu', 'refine.cu', 'gridbag.cu', 'mil.cu', 'p2p.cu', 'nms.cu', 'conv_tc.cu', 'tower_bwd.cu', 'wgrad_tc.cu', 'assign.cu', 'lsap.cu', 'rpn.cu', 'loss_bwd.cu', 'roi_align.cu']
 ARCH = ['-gencode', 'arch=compute_100a,code=sm_100a']
 FLAGS = ['-O3', '-std=c++17', '-lineinfo', '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr', '-Xptxas', '-v']
 

@@ -538,14 +538,6 @@ gn_relu_apply_kernel(const float4* __restrict__ y, const double* __restrict__ st
 }
 
 // ---- fp16 two-term split (split_h2, tc_ptx.cuh) ----
-// power-of-two scale that brings amax into [2^11, 2^12) (fp16 max is 65504; small values keep 3e-8*|scale| absolute precision)
-__device__ __forceinline__ float pow2_scale_for(float amax) {
-  if (!(amax > 0.f) || !isfinite(amax)) return 1.f;
-  int e;
-  frexpf(amax, &e);                 // amax = m * 2^e, m in [0.5, 1)
-  return ldexpf(1.f, 12 - e);       // amax*scale in [2^11, 2^12)
-}
-
 __device__ __forceinline__ float amax4(float m, const float4 v) {
   return fmaxf(m, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
 }
@@ -944,6 +936,19 @@ extern "C" int ptb_split_f16(const float* x, int64_t n, int auto_scale, void* hi
   split_f16_kernel<<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(x), n / 4, amax, reinterpret_cast<uint2*>(hi),
                                                     reinterpret_cast<uint2*>(lo), dev_inv_scale);
   return check_launch("ptb_split_f16");
+}
+
+extern "C" int ptb_amax_abs(const float* x, int64_t n, unsigned int* dev_amax_bits, int accumulate, void* stream) {
+  PTB_REQUIRE(n >= 0 && n % 4 == 0, "n must be a multiple of 4");
+  PTB_REQUIRE(((uintptr_t)x % 16 == 0) && dev_amax_bits, "alignment / NULL");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!accumulate && cudaMemsetAsync(dev_amax_bits, 0, 4, st) != cudaSuccess) return fail("%s", "ptb_amax_abs: cudaMemsetAsync failed");
+  if (n == 0) return 0;
+  long long blocks = (n / 4 + 255) / 256;
+  const long long cap = (long long)sm_count() * 16;
+  if (blocks > cap) blocks = cap;
+  amax_abs_kernel<<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(x), n / 4, dev_amax_bits);
+  return check_launch("ptb_amax_abs");
 }
 
 extern "C" int ptb_split_f16_amax(const float* x, int64_t n, const unsigned int* dev_amax_bits, void* hi, void* lo,

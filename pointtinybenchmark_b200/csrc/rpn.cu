@@ -19,6 +19,7 @@
 // Levels are disjoint after the level offset because every candidate box is clipped to [0, img_w] x [0, img_h] (>= 0), so the
 // joint greedy NMS of the reference decomposes per level exactly.  Everything here is latency / HBM-scan work (1.3 MB of logits
 // per image at configs[3]); the design goal is one pass over the logits and no intermediate anchor / IoU tensors.
+#include "bbox_coder.cuh"
 #include "ptb_common.cuh"
 #include "topk_select.cuh"
 #include <math_constants.h>
@@ -71,11 +72,6 @@ rpn_score_kernel(const float* __restrict__ cls /*[B][A][H][W]*/, int B, int A, i
   }
 }
 
-struct DecodeCfg {
-  float mean[4], stdv[4];
-  float max_ratio;
-};
-
 __global__ void __launch_bounds__(256)
 rpn_decode_kernel(const float* __restrict__ bbox /*[B][4A][H][W]*/, const float* __restrict__ key /*[B][Q]*/,
                   const int32_t* sel /*[B][Ptot] (level segment filled; may alias cand_idx)*/, int B, int A, int H, int W,
@@ -95,24 +91,8 @@ rpn_decode_kernel(const float* __restrict__ bbox /*[B][4A][H][W]*/, const float*
   const float ax1 = __fadd_rn(base[4 * a], fx), ay1 = __fadd_rn(base[4 * a + 1], fy);
   const float ax2 = __fadd_rn(base[4 * a + 2], fx), ay2 = __fadd_rn(base[4 * a + 3], fy);
   const float* d = bbox + ((size_t)b * 4 * A + 4 * a) * HW + cell;
-  // delta_xywh_bbox_coder.py:209-246 (fp32, separate multiply and add as ATen executes them)
-  const float dx = __fadd_rn(__fmul_rn(d[0], dc.stdv[0]), dc.mean[0]);
-  const float dy = __fadd_rn(__fmul_rn(d[(size_t)HW], dc.stdv[1]), dc.mean[1]);
-  float dw = __fadd_rn(__fmul_rn(d[2 * (size_t)HW], dc.stdv[2]), dc.mean[2]);
-  float dh = __fadd_rn(__fmul_rn(d[3 * (size_t)HW], dc.stdv[3]), dc.mean[3]);
-  const float px = __fmul_rn(__fadd_rn(ax1, ax2), 0.5f), py = __fmul_rn(__fadd_rn(ay1, ay2), 0.5f);
-  const float pw = __fsub_rn(ax2, ax1), ph = __fsub_rn(ay2, ay1);
-  const float dxw = __fmul_rn(pw, dx), dyh = __fmul_rn(ph, dy);
-  dw = fminf(fmaxf(dw, -dc.max_ratio), dc.max_ratio);
-  dh = fminf(fmaxf(dh, -dc.max_ratio), dc.max_ratio);
-  const float gw = __fmul_rn(pw, expf(dw)), gh = __fmul_rn(ph, expf(dh));
-  const float gx = __fadd_rn(px, dxw), gy = __fadd_rn(py, dyh);
-  const float hw2 = __fmul_rn(gw, 0.5f), hh2 = __fmul_rn(gh, 0.5f);
-  float x1 = __fsub_rn(gx, hw2), y1 = __fsub_rn(gy, hh2), x2 = __fadd_rn(gx, hw2), y2 = __fadd_rn(gy, hh2);
   const float mw = (float)img_hw[2 * b + 1], mh = (float)img_hw[2 * b];      // max_shape = img_shape[:2] flipped -> (w, h)
-  x1 = x1 < 0.f ? 0.f : x1; y1 = y1 < 0.f ? 0.f : y1; x2 = x2 < 0.f ? 0.f : x2; y2 = y2 < 0.f ? 0.f : y2;
-  x1 = x1 > mw ? mw : x1; y1 = y1 > mh ? mh : y1; x2 = x2 > mw ? mw : x2; y2 = y2 > mh ? mh : y2;
-  cand_box[o] = make_float4(x1, y1, x2, y2);
+  cand_box[o] = delta2bbox_clip(ax1, ay1, ax2, ay2, d[0], d[(size_t)HW], d[2 * (size_t)HW], d[3 * (size_t)HW], dc, mw, mh);
   cand_score[o] = key[(size_t)b * HW * A + q];
   cand_idx[o] = q;
 }

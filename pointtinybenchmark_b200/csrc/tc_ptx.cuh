@@ -189,6 +189,14 @@ __device__ __forceinline__ void split_h2(float v, __half& h, __half& l) {
   l = __float2half_rn(v - __half2float(h));
 }
 
+// power-of-two scale that brings amax into [2^11, 2^12) (fp16 max is 65504; small values keep 3e-8*|scale| absolute precision)
+__device__ __forceinline__ float pow2_scale_for(float amax) {
+  if (!(amax > 0.f) || !isfinite(amax)) return 1.f;
+  int e;
+  frexpf(amax, &e);                 // amax = m * 2^e, m in [0.5, 1)
+  return ldexpf(1.f, 12 - e);       // amax*scale in [2^11, 2^12)
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);

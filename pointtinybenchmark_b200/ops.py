@@ -850,3 +850,121 @@ def conv_tc_f16(x_h, x_l, packed, taps, n_out, bias=None, dev_out_scale=None, ld
     check(lib.ptb_conv_tc_f16x2(_ptr(x_h), _ptr(x_l), _ptr(w_h), _ptr(w_l), B, H, W, Cin, taps, n_out, n_mma, float(inv_w),
                                 _ptr(dev_out_scale), _ptr(bias), _ptr(y), ldy, _stream()), 'ptb_conv_tc_f16x2')
     return y
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# R-CNN box stage (roi_head.py)
+# ----------------------------------------------------------------------------------------------------------------------
+def amax_abs(tensors):
+    """ptb_amax_abs over several fp32 tensors -> (1,) int32 device tensor holding the float bits of max|x| (no host sync)."""
+    lib = _lib.load()
+    bits = torch.empty(1, dtype=torch.int32, device=tensors[0].device)
+    for i, t in enumerate(tensors):
+        _chk(t, torch.float32, 'x')
+        check(lib.ptb_amax_abs(_ptr(t), t.numel(), _ptr(bits), 1 if i else 0, _stream()), 'ptb_amax_abs')
+    return bits
+
+
+def roi_align(feats_nhwc, rois, out_size=(7, 7), spatial_scales=None, sampling_ratio=0, aligned=True, finest_scale=56, f16_pair=False,
+              row_multiple=16, want_levels=False):
+    """ptb_roi_align.  feats_nhwc: list of (B,H,W,C) contiguous fp32 level maps; rois (M,5) fp32.
+    returns fp32 (M, oh, ow, C) — or with f16_pair (h, l, dev_inv_scale), h / l (M_pad, oh*ow*C) fp16, M_pad = M rounded up to
+    row_multiple — plus the (M,) int8 levels when want_levels."""
+    lib = _lib.load()
+    L = len(feats_nhwc)
+    if not 1 <= L <= 5:
+        raise ValueError(f'ptb_roi_align takes 1 to 5 levels, got {L}')
+    for f in feats_nhwc:
+        _chk(f, torch.float32, 'feat')
+    _chk(rois, torch.float32, 'rois')
+    if rois.dim() != 2 or rois.shape[1] != 5:
+        raise ValueError('rois must be (M, 5)')
+    B, _, _, C = feats_nhwc[0].shape
+    if any(f.shape[0] != B or f.shape[3] != C for f in feats_nhwc):
+        raise ValueError('level maps must share batch size and channels')
+    if C % 32:
+        raise ValueError(f'ptb_roi_align needs C % 32 == 0, got C = {C}')
+    oh, ow = out_size
+    M = rois.shape[0]
+    dev = rois.device
+    hw = (ctypes.c_int32 * (2 * L))(*[int(v) for f in feats_nhwc for v in f.shape[1:3]])
+    fp = (ctypes.c_void_p * L)(*[f.data_ptr() for f in feats_nhwc])
+    sc = (ctypes.c_float * L)(*[float(s) for s in spatial_scales])
+    lvl = torch.empty(M, dtype=torch.int8, device=dev) if want_levels else None
+    if f16_pair:
+        Mp = (M + row_multiple - 1) // row_multiple * row_multiple
+        bits = amax_abs(feats_nhwc)
+        h = torch.empty((Mp, oh * ow * C), dtype=torch.float16, device=dev)
+        l = torch.empty_like(h)
+        inv = torch.empty(1, dtype=torch.float32, device=dev)
+        check(lib.ptb_roi_align(_ptr(rois), M, Mp, fp, hw, sc, L, B, C, oh, ow, int(sampling_ratio), 1 if aligned else 0, float(finest_scale),
+                                _ptr(bits), None, _ptr(h), _ptr(l), _ptr(inv), _ptr(lvl), _stream()), 'ptb_roi_align')
+        out = (h, l, inv)
+    else:
+        out = torch.empty((M, oh, ow, C), dtype=torch.float32, device=dev)
+        check(lib.ptb_roi_align(_ptr(rois), M, M, fp, hw, sc, L, B, C, oh, ow, int(sampling_ratio), 1 if aligned else 0, float(finest_scale),
+                                None, _ptr(out), None, None, None, _ptr(lvl), _stream()), 'ptb_roi_align')
+    return (out, lvl) if want_levels else out
+
+
+def relu_split_f16(y, n=None, overflow_flag=None):
+    """ptb_relu_split_f16: (rows, ld) fp32 -> fp16 pair (rows, n) of relu(y[:, :n]) at unit scale."""
+    lib = _lib.load()
+    _chk(y, torch.float32, 'y')
+    rows, ld = y.shape
+    n = ld if n is None else n
+    h = torch.empty((rows, n), dtype=torch.float16, device=y.device)
+    l = torch.empty_like(h)
+    check(lib.ptb_relu_split_f16(_ptr(y), rows, n, ld, _ptr(h), _ptr(l), _ptr(overflow_flag), _stream()), 'ptb_relu_split_f16')
+    return h, l
+
+
+def linear_tc_f16(x_h, x_l, packs, n_out, bias=None, dev_in_scale=None):
+    """y (M_pad, ldy) = x @ W.T + bias on ptb_conv_tc_f16x2 with 1 tap: the rows of x (M_pad, K) fp16 pair are the 'pixels' of a
+    (1, M_pad/16, 16, K) operand; `packs` = [(h, l, inv_w, n_mma)] column slices of <= 256 outputs (conv_tc_pack_weight_f16)."""
+    lib = _lib.load()
+    _chk(x_h, torch.float16, 'x_h'); _chk(x_l, torch.float16, 'x_l')
+    Mp, K = x_h.shape
+    if Mp % 16 or K % 32:
+        raise ValueError(f'linear_tc_f16: rows must be a multiple of 16 and K of 32, got {tuple(x_h.shape)}')
+    ldy = (n_out + 3) // 4 * 4
+    y = torch.empty((Mp, ldy), dtype=torch.float32, device=x_h.device)
+    if Mp == 0:
+        return y
+    n0 = 0
+    for (w_h, w_l, inv_w, n_mma) in packs:
+        ns = min(n_mma, n_out - n0)
+        check(lib.ptb_conv_tc_f16x2(_ptr(x_h), _ptr(x_l), _ptr(w_h), _ptr(w_l), 1, Mp // 16, 16, K, 1, ns, n_mma, float(inv_w),
+                                    _ptr(dev_in_scale), _ptr(bias[n0:] if bias is not None else None), ctypes.c_void_p(y.data_ptr() + 4 * n0),
+                                    ldy, _stream()), 'ptb_conv_tc_f16x2')
+        n0 += ns
+    return y
+
+
+def rcnn_bbox_decode(rois, n_per_img, cls, reg, num_classes, means, stds, img_hw, scale_factor=None, mask_padding=False,
+                     wh_ratio_clip=16 / 1000, want_scores=True, want_candidates=True):
+    """ptb_rcnn_bbox_decode.  rois (B*n, 5); cls (B*n, >= N+1) / reg (B*n, >= 4N) row-strided views with unit inner stride.
+    returns boxes (B*n, 4N), scores (B*n, N+1) | None, candidate scores (B, n*N, N) | None."""
+    lib = _lib.load()
+    _chk(rois, torch.float32, 'rois'); _chk(img_hw, torch.int32, 'img_hw')
+    for t, nm in ((cls, 'cls'), (reg, 'reg')):
+        if t.dtype != torch.float32 or not t.is_cuda or t.stride(-1) != 1:
+            raise RuntimeError(f'{nm}: expected a CUDA fp32 matrix with unit inner stride')
+    if scale_factor is not None:
+        _chk(scale_factor, torch.float32, 'scale_factor')
+    R = rois.shape[0]
+    B = img_hw.shape[0]
+    if R != B * n_per_img:
+        raise ValueError('rois must hold n_per_img rows per image')
+    N = int(num_classes)
+    dev = rois.device
+    boxes = torch.empty((R, 4 * N), dtype=torch.float32, device=dev)
+    scores = torch.empty((R, N + 1), dtype=torch.float32, device=dev) if want_scores else None
+    cand = torch.empty((B, n_per_img * N, N), dtype=torch.float32, device=dev) if want_candidates else None
+    mean = (ctypes.c_float * 4)(*[float(v) for v in means])
+    std = (ctypes.c_float * 4)(*[float(v) for v in stds])
+    check(lib.ptb_rcnn_bbox_decode(_ptr(rois), B, n_per_img, _ptr(cls), cls.stride(0) if R > 1 else cls.shape[1], _ptr(reg),
+                                   reg.stride(0) if R > 1 else reg.shape[1], N, 1 if mask_padding else 0, mean, std, float(wh_ratio_clip),
+                                   _ptr(img_hw), _ptr(scale_factor), _ptr(boxes), _ptr(scores), _ptr(cand), _stream()),
+          'ptb_rcnn_bbox_decode')
+    return boxes, scores, cand

@@ -86,3 +86,24 @@ def build_sampler(cfg, **default_args):
 
 def build_anchor_generator(cfg, default_args=None):
     return ANCHOR_GENERATORS.build(cfg, default_args)
+
+
+# ---- R-CNN box stage (roi_head.py): RoI extractors have their own registry in mmdet (mmdet/models/builder.py)
+try:   # pragma: no cover
+    from mmdet.models.builder import ROI_EXTRACTORS as _R
+    ROI_EXTRACTORS = _R
+except Exception:
+    ROI_EXTRACTORS = Registry('roi_extractor')
+
+
+def register_roi_heads():
+    """register SingleRoIExtractor into ROI_EXTRACTORS and Shared2FCBBoxHead / StandardRoIHead into HEADS (force=True over the reference
+    classes when mmdet is importable)."""
+    from .roi_head import Shared2FCBBoxHead, SingleRoIExtractor, StandardRoIHead
+    ROI_EXTRACTORS.register_module(name='SingleRoIExtractor', force=True, module=SingleRoIExtractor)
+    for c in (Shared2FCBBoxHead, StandardRoIHead):
+        HEADS.register_module(name=c.__name__, force=True, module=c)
+
+
+def build_roi_extractor(cfg, default_args=None):
+    return ROI_EXTRACTORS.build(cfg, default_args)
